@@ -15,7 +15,7 @@ than L2 or stated otherwise; each with the CPU oracle beside it):
   config5         100 KF / 20k LM / 300k obs window: one GPU, and -- when launched on N > 1 ranks -- the landmark-sharded
                   solve with the NCCL all-reduce of the reduced system, checked against the one-GPU solve (row 5)
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--no-sub]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--no-sub] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -121,6 +121,43 @@ def measured_peak():
         with open(p) as f:
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_LIMIT_BYTES = 60 * 10**6  # array data of --dump-outputs: with the .npy headers, below 64 MB
+SOLVE_FIELDS = ("initial_cost", "final_cost", "num_iterations", "num_successful_steps", "termination", "num_landmarks",
+                "num_residual_blocks")
+
+
+def dump_outputs(out_dir, results, windows):
+    """Writes what a caller of the resident batch solve receives, one DIR/<name>.npy per array (float64; the rejection flags
+    as float32), windows stacked along the first axis in batch order, so that two builds can be compared output for output.
+    solve_<field> holds the summary of every inner solve, zero past num_solves.  When the whole batch would exceed
+    DUMP_LIMIT_BYTES, a fixed, seeded sample of whole windows is written; window_index names the windows kept."""
+    from limo_b200.capi_types import KBA_MAX_SOLVES
+    arrays = {
+        "kf_pose": np.stack([r.kf_pose for r in results]),
+        "kf_plane": np.stack([r.kf_plane for r in results]),
+        "lm_pos": np.stack([r.lm_pos[:w.n_lm] for r, w in zip(results, windows)]),
+        "lm_rejected": np.stack([r.lm_rejected[:w.n_lm] for r, w in zip(results, windows)]).astype(np.float32),
+        "status": np.array([r.c.status for r in results], dtype=np.float64),
+        "num_solves": np.array([r.c.num_solves for r in results], dtype=np.float64),
+        "initial_cost": np.array([r.c.initial_cost for r in results]),
+        "final_cost": np.array([r.c.final_cost for r in results]),
+        "window_index": np.arange(len(results), dtype=np.float64),
+    }
+    for f in SOLVE_FIELDS:
+        a = np.zeros((len(results), KBA_MAX_SOLVES))
+        for i, r in enumerate(results):
+            a[i, :r.c.num_solves] = [getattr(s, f) for s in r.solves]
+        arrays["solve_" + f] = a
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = DUMP_LIMIT_BYTES * len(results) // total
+        idx = np.sort(np.random.default_rng(0).choice(len(results), keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -397,7 +434,12 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=6, help="window solves timed for cpu_baseline (~0.5 s each); 0 = skip the CPU legs")
     ap.add_argument("--in-flight", type=int, default=4, help="steps in flight of the end-to-end measurement (handles / streams)")
     ap.add_argument("--no-sub", action="store_true", help="headline only: skip the sub-records of configs 3, 4, 5 and the batch sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step (rank 0's windows) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 arm")
 
     from limo_b200 import parallel
     rank, local_rank, world = parallel.rank_info()
@@ -450,6 +492,8 @@ def main():
     cnt = h.counters(reset=True)
     h.enable_kernel_timing(False)
     results = batch.download()
+    if args.dump_outputs and rank == 0:  # before the end-to-end steps below reuse these result buffers
+        dump_outputs(args.dump_outputs, results, windows)
     done = all(r.c.status == 0 for r in results)
     converged = all(r.solves[r.c.num_solves - 1].termination == 0 for r in results)  # KBA_TERM_CONVERGENCE of the final solve
     iters = [sum(s.num_iterations for s in r.solves) for r in results]
